@@ -94,6 +94,25 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_LIMIT = 64 << 20   # bytes written by --dump-outputs at most
+
+
+def dump_outputs(dirname, arrays, seed=0):
+    """Write each float tensor as dirname/<name>.npy in float32 so that two builds can be compared output for output.
+    When the arrays together exceed DUMP_LIMIT, each is replaced by the same fixed, seeded sample of its flattened
+    elements (sorted positions; the sample depends only on the array's size and `seed`)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT:
+            keep = max(1, a.size * DUMP_LIMIT // total)
+            idx = np.sort(np.random.default_rng(seed).choice(a.size, keep, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def build_info():
     d = {}
     try:
@@ -482,6 +501,8 @@ def run_b200(args):
     launches = launch_total() - l0
     value = B_glob * args.steps / (ms_total / 1000.0)
     assert all(torch.isfinite(o).all() for o in outs)
+    if args.dump_outputs:   # x0 of the last timed step: this rank's images in global order
+        dump_outputs(args.dump_outputs, {"x0" if world == 1 else "x0_rank%d" % rank: torch.cat(outs)})
 
     # ---- (2) end to end through the public API with HOST buffers (pinned): H2D of the inputs, the sampler exactly as
     #          test.py drives it (UNet workloads: torch RNG, one randn_like per step), D2H of x0, the final gather
@@ -571,7 +592,10 @@ def main():
     ap.add_argument("--no-tf32", action="store_true", help="reference arm on cuda: disable cuDNN/cuBLAS TF32")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="B200 arm: write x0 of the last timed step as DIR/x0.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,6 +1,5 @@
 """Golden fixture for the Refusion latent autoencoder UNet.encode/decode, generated from the imported reference
-(random small configuration; the shipped checkpoint latent-dehazing.pth is exercised by a CPU test when the reference
-checkout is present).    python tests/golden/make_golden_latent.py"""
+(random small configuration).    python tests/golden/make_golden_latent.py"""
 import importlib.util
 import os
 import sys

@@ -139,12 +139,40 @@ def test_sharded_gather_gloo_world2():
     assert torch.equal(res[0][2], res[1][2]) and res[0][2].abs().sum() > 0
 
 
-def test_launcher_patches_reference_tree():
-    """Drop-in mechanics (INTEGRATION.md 1): on a checkout of the reference, `run.install` swaps the sampler and
-    network classes the reference scripts resolve by name.  Needs the reference tree (absent on the GPU box)."""
-    ref = "/root/reference/codes/config/deraining"
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not available")
+def _reference_layout_tree(root):
+    """A minimal tree with the reference's package layout as the launcher sees it: `codes/utils` re-exports the samplers
+    of `utils/sde_utils.py`; `codes/config/deraining/models/networks.py` builds the network with
+    `getattr(models.modules, which_model_G)(**setting)` (networks.py:10-15); `models.modules` exports the PyTorch
+    ConditionalUNet (forward(xt, cond, time)) and ConditionalNAFNet."""
+    files = {
+        "codes/utils/__init__.py": "from .sde_utils import *\n",
+        "codes/utils/sde_utils.py": "class IRSDE:\n    pass\n\n\nclass DenoisingSDE:\n    pass\n",
+        "codes/config/deraining/models/__init__.py": "",
+        "codes/config/deraining/models/networks.py": (
+            "from models import modules as M\n\n\n"
+            "def define_G(opt):\n"
+            "    net = opt['network_G']\n"
+            "    return getattr(M, net['which_model_G'])(**net['setting'])\n"),
+        "codes/config/deraining/models/modules/__init__.py": (
+            "import torch\n\n\n"
+            "class ConditionalUNet(torch.nn.Module):\n"
+            "    def forward(self, xt, cond, time):\n"
+            "        raise AssertionError('the PyTorch network must not be used')\n\n\n"
+            "class ConditionalNAFNet(ConditionalUNet):\n"
+            "    pass\n"),
+    }
+    for rel, text in files.items():
+        path = os.path.join(root, rel)
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, "w") as f:
+            f.write(text)
+    return os.path.join(root, "codes", "config", "deraining")
+
+
+def test_launcher_patches_reference_tree(tmp_path):
+    """Drop-in mechanics (INTEGRATION.md 1): on a tree laid out like the reference's, `run.install` swaps the sampler and
+    network classes the reference scripts resolve by name."""
+    ref = _reference_layout_tree(str(tmp_path))
     import subprocess
     import sys
     code = (

@@ -124,50 +124,6 @@ def test_latent_unet_oracle_vs_reference():
     assert list(shapes) == list(g["state"])
 
 
-def test_latent_unet_oracle_real_checkpoint():
-    """The shipped latent-dehazing.pth (2.0 M params) through the reference module vs the oracle (needs the reference)."""
-    import os
-    import sys
-    ck = "/root/reference/codes/config/latent-dehazing/pretrained_models/latent-dehazing.pth"
-    if not os.path.exists(ck):
-        import pytest
-        pytest.skip("reference checkout not available")
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    from make_golden_latent import load_unet_arch
-    arch = load_unet_arch()
-    sd = torch.load(ck, map_location="cpu", weights_only=True)
-    net = arch.UNet(in_ch=3, out_ch=3, ch=8, ch_mult=[4, 8, 8, 16], embed_dim=8).eval()
-    net.load_state_dict(sd, strict=True)
-    x = torch.rand(1, 3, 50, 70, generator=torch.Generator().manual_seed(0))
-    with torch.no_grad():
-        z, h = net.encode(x)
-        y = net.decode(z, h)
-    zo, ho = O.latent_unet_encode(sd, x, [4, 8, 8, 16])
-    _close(zo, z, 1e-4)
-    for a, b in zip(ho, h):
-        _close(a, b, 1e-3)
-    # decode is NOT compared for this checkpoint: on such inputs the reference's own fp32 and fp64 decodes differ by
-    # O(100) (ill-conditioned trained weights), so no fp32 restatement can be pinned there; decode parity is pinned on
-    # the well-conditioned random-weight fixture (test_latent_unet_oracle_vs_reference).
-    assert y.shape == x.shape
-    assert list(O.latent_unet_param_shapes(3, 3, 8, [4, 8, 8, 16], 8)) == list(sd)
-    # A natural image (images/1.png crop): the oracle follows the reference's fp32 op order closely enough to reproduce
-    # its decode to 1e-5 of the output range, although that range is ~78 and the reference's fp32 and fp64 runs differ by
-    # 0.17 in z and ~67 in y here - the checkpoint is ill-conditioned, so this pins the restatement, not a tolerance a
-    # re-ordered fp32 implementation (the GPU kernels) can be held to.
-    import cv2
-    import numpy as np
-    img = cv2.imread("/root/reference/images/1.png")
-    xi = torch.from_numpy(img[:, :, [2, 1, 0]].astype(np.float32) / 255.).permute(2, 0, 1)[None][:, :, :160, :224].contiguous()
-    with torch.no_grad():
-        zi, hi = net.encode(xi)
-        yi = net.decode(zi, hi)
-    zo, ho = O.latent_unet_encode(sd, xi, [4, 8, 8, 16])
-    yo = O.latent_unet_decode(sd, zo, ho, [4, 8, 8, 16], 160, 224)
-    _close(zo, zi, 1e-4)
-    assert (yo - yi).abs().max().item() < 1e-4 * yi.abs().max().item()
-
-
 # ---- image helpers (oracle/imaging_oracle.py vs the reference's img_utils outputs) ---------------------------
 def _imaging_golden():
     import os
