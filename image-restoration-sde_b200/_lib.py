@@ -19,7 +19,7 @@ NUM_COEF = 8
 FLAG_FORCE_SIMT = 1   # irsde_config.flags: bf16 storage through the SIMT conv engine (debug aid)
 
 # every symbol include/irsde_b200.h declares
-SYMBOLS = ["irsde_create", "irsde_create_ch_mult", "irsde_create_nafnet", "irsde_create_latent_unet", "irsde_latent_shape", "irsde_latent_encode",
+SYMBOLS = ["irsde_create", "irsde_create_ch_mult", "irsde_create_nafnet", "irsde_create_nafnet_lens", "irsde_set_lens", "irsde_create_latent_unet", "irsde_latent_shape", "irsde_latent_encode",
            "irsde_latent_decode", "irsde_tensor2img_u8", "irsde_img2tensor_u8", "irsde_sqerr_u8", "irsde_ssim_workspace", "irsde_ssim_u8", "irsde_destroy", "irsde_last_error", "irsde_version", "irsde_load_tensor",
            "irsde_finalize_weights", "irsde_set_schedule", "irsde_set_coeffs", "irsde_noise_fn", "irsde_step",
            "irsde_reverse", "irsde_noise_state", "irsde_noise_state_images", "irsde_set_image_base", "irsde_set_image_uids", "irsde_comm_unique_id", "irsde_comm_init", "irsde_broadcast_weights", "irsde_gather", "irsde_launch_count", "irsde_device_bytes", "irsde_conv2d", "irsde_profile_begin",
@@ -102,6 +102,8 @@ def load():
     L.irsde_gather.restype = ctypes.c_int
     L.irsde_random_states.argtypes = [vp, vp, vp, vp, vp, vp, i32, i64, vp]
     L.irsde_random_states.restype = ctypes.c_int
+    L.irsde_set_lens.argtypes = [vp, fp, i32, vp]
+    L.irsde_set_lens.restype = ctypes.c_int
     L.irsde_trim.argtypes = [vp]
     L.irsde_trim.restype = ctypes.c_int
     L.irsde_profile_begin.argtypes = [vp]

@@ -21,6 +21,7 @@
 
 #include "../../include/irsde_b200.h"
 #include "common.cuh"
+#include "nafnet.cuh"
 
 using namespace irsde;
 
@@ -44,6 +45,8 @@ struct RunCfg {  // per-invocation pointers read by the op closures at launch ti
   const float* ss = nullptr;  // time-modulation table
   const int* t_ptr = nullptr;
   int ss_img_stride = 0;
+  const float* cam = nullptr;  // lens network: camera table [rows][cam_S] (irsde_set_lens)
+  int cam_img_stride = 0;
 };
 
 struct Plan;
@@ -77,6 +80,9 @@ struct Plan {
   int chain_cap = 0;
   cudaGraphExec_t graph[IRSDE_NUM_MODES] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   long long step_launches[IRSDE_NUM_MODES] = {0, 0, 0, 0, 0};
+  // camera table pointer / image stride a step graph was captured with (lens network): a change re-captures
+  const float* graph_cam[IRSDE_NUM_MODES] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+  int graph_cam_stride[IRSDE_NUM_MODES] = {0, 0, 0, 0, 0};
   long long bytes = 0;               // device memory owned by this plan (plan cache accounting)
   unsigned long long last_use = 0;   // LRU stamp
 };
@@ -87,6 +93,7 @@ struct NafCfg {
   int img_channel = 0, width = 0, middle = 0, n_enc = 0, n_dec = 0;
   int enc[8] = {0}, dec[8] = {0};
   bool latent = false;
+  bool lens = false;  // latent-bokeh variant: time_mlp.0/.2 keys, camera-modulated FFN gate, plain ending(x)
 };
 
 // Refusion latent autoencoder UNet (codes/config/latent-dehazing/models/modules/UNet_arch.py:17-97)
@@ -133,6 +140,15 @@ struct irsde_ctx {
   std::vector<ProfEv> prof_events;
   bool use_tc = false;  // bf16 mode: route eligible convs through the tcgen05 engine
   std::vector<int> udim;  // UNet channels per level: nf * [1, ch_mult...] (DenoisingUNet_arch.py:51-56)
+  // lens network (irsde_create_nafnet_lens): every block's cam_mlp.1 concatenated [cam_S][2w], and the per-image camera
+  // table cam_table[lens_n][cam_S] = (cam_scale, cam_shift) of every block, computed by irsde_set_lens.  Captured step graphs
+  // read cam_table, so it is only re-written after draining the device and only re-allocated when it must grow.
+  std::map<std::string, int> cam_off;
+  int cam_S = 0;
+  float *cam_wall = nullptr, *cam_ball = nullptr;
+  float *cam_table = nullptr, *cam_gate = nullptr, *lens_dev = nullptr;
+  int lens_cap = 0, lens_n = 0;
+  std::vector<float> lens_host;  // [lens_n][3] as last set
 };
 
 namespace {
@@ -333,10 +349,19 @@ std::vector<NafBlockInfo> naf_blocks(const NafCfg& n) {
 std::vector<ParamSpec> naf_param_specs(const NafCfg& n) {
   std::vector<ParamSpec> v;
   int64_t w = n.width, td = 4 * w, ic = n.img_channel;
-  v.push_back({"time_mlp.1.weight", {2 * td, w}});
-  v.push_back({"time_mlp.1.bias", {2 * td}});
-  v.push_back({"time_mlp.3.weight", {td, td}});
-  v.push_back({"time_mlp.3.bias", {td}});
+  // lens variant (latent-bokeh/.../DenoisingNAFNet_arch.py:102-113): time_mlp without the embedding module (.0/.2), cam_mlp
+  const char* tm = n.lens ? "time_mlp.0." : "time_mlp.1.";
+  const char* tm2 = n.lens ? "time_mlp.2." : "time_mlp.3.";
+  v.push_back({std::string(tm) + "weight", {2 * td, w}});
+  v.push_back({std::string(tm) + "bias", {2 * td}});
+  v.push_back({std::string(tm2) + "weight", {td, td}});
+  v.push_back({std::string(tm2) + "bias", {td}});
+  if (n.lens) {
+    v.push_back({"cam_mlp.0.weight", {2 * td, 3 * w}});
+    v.push_back({"cam_mlp.0.bias", {2 * td}});
+    v.push_back({"cam_mlp.2.weight", {td, td}});
+    v.push_back({"cam_mlp.2.bias", {td}});
+  }
   v.push_back({"intro.weight", {w, 2 * ic, 3, 3}});
   v.push_back({"intro.bias", {w}});
   v.push_back({"ending.weight", {ic, w, 3, 3}});
@@ -346,8 +371,13 @@ std::vector<ParamSpec> naf_param_specs(const NafCfg& n) {
     const std::string& p = blk.pre;
     v.push_back({p + "beta", {1, c, 1, 1}});
     v.push_back({p + "gamma", {1, c, 1, 1}});
-    v.push_back({p + "mlp.1.weight", {4 * c, td / 2}});
-    v.push_back({p + "mlp.1.bias", {4 * c}});
+    const std::string mp = p + (n.lens ? "time_mlp.1." : "mlp.1.");
+    v.push_back({mp + "weight", {4 * c, td / 2}});
+    v.push_back({mp + "bias", {4 * c}});
+    if (n.lens) {  // latent-bokeh/.../DenoisingNAFNet_arch.py:22-24
+      v.push_back({p + "cam_mlp.1.weight", {2 * c, td / 2}});
+      v.push_back({p + "cam_mlp.1.bias", {2 * c}});
+    }
     v.push_back({p + "conv1.weight", {2 * c, c, 1, 1}});
     v.push_back({p + "conv1.bias", {2 * c}});
     v.push_back({p + "conv2.weight", {2 * c, 1, 3, 3}});
@@ -1008,11 +1038,21 @@ struct Builder {
     conv(pre + "conv4.weight", V{t1, c, c}, H, W, 1, 1, 0, 1, b4.c_str(), "", 0, nullptr, V{t2, 2 * c, 2 * c}, 2 * c);
     release(t1);
     g = tmp(npix * c);
-    plan->ops.push_back(OpRec{CAT_MISC, 0.0, [=](Plan*, cudaStream_t st) {
-      launch_simple_gate<T>(t2, 2 * c, g, c, npix, c, st);
-      cx->launches++;
-    }});
-    plan->ops.back().label = pre + "simple_gate";
+    if (ctx->naf.lens) {  // x = SimpleGate(x) * (cam_scale + 1) + cam_shift   (latent-bokeh/.../DenoisingNAFNet_arch.py:82-83)
+      const int coff = ctx->cam_off[pre], cS = ctx->cam_S;
+      plan->ops.push_back(OpRec{CAT_MISC, 0.0, [=](Plan* p, cudaStream_t st) {
+        CamMod m{p->cur.cam, cS, coff, p->cur.cam_img_stride, N};
+        launch_simple_gate<T>(t2, 2 * c, g, c, npix, c, st, m, B);
+        cx->launches++;
+      }});
+      plan->ops.back().label = pre + "simple_gate+cam";
+    } else {
+      plan->ops.push_back(OpRec{CAT_MISC, 0.0, [=](Plan*, cudaStream_t st) {
+        launch_simple_gate<T>(t2, 2 * c, g, c, npix, c, st);
+        cx->launches++;
+      }});
+      plan->ops.back().label = pre + "simple_gate";
+    }
     release(t2);
     std::string b5 = pre + "conv5.bias";
     pending_mult = fw(pre + "gamma");
@@ -1375,8 +1415,9 @@ int upload_coeffs(irsde_ctx* ctx, int mode, const float* tab, int T) {
 // times[rows] -> table[rows][S] for either network family
 void time_rows(irsde_ctx* ctx, const float* times, int rows, float* temb_ws, float* table, cudaStream_t st) {
   if (ctx->naf.on) {
-    launch_naf_time_gate(times, rows, ctx->naf.width, ctx->raw["time_mlp.1.weight"].dev, ctx->raw["time_mlp.1.bias"].dev,
-                         ctx->raw["time_mlp.3.weight"].dev, ctx->raw["time_mlp.3.bias"].dev, temb_ws, st);
+    const std::string a = ctx->naf.lens ? "time_mlp.0." : "time_mlp.1.", b = ctx->naf.lens ? "time_mlp.2." : "time_mlp.3.";
+    launch_naf_time_gate(times, rows, ctx->naf.width, ctx->raw[a + "weight"].dev, ctx->raw[a + "bias"].dev,
+                         ctx->raw[b + "weight"].dev, ctx->raw[b + "bias"].dev, temb_ws, st);
     launch_time_rows(temb_ws, rows, 2 * ctx->naf.width, ctx->wall, ctx->ball, ctx->S, table, st);
   } else {
     launch_time_table(times, rows, ctx->cfg.nf, ctx->raw["time_mlp.1.weight"].dev, ctx->raw["time_mlp.1.bias"].dev,
@@ -1404,6 +1445,31 @@ int ensure_chain_table(irsde_ctx* ctx, Plan* p, int T, cudaStream_t st) {
       if (p->graph[m]) { cudaGraphExecDestroy(p->graph[m]); p->graph[m] = nullptr; }
   }
   time_rows(ctx, p->chain_times, rows, p->chain_temb, p->chain_table, st);
+  return IRSDE_OK;
+}
+
+// lens network: lens_host [lens_n][3] -> cam_table [lens_n][cam_S].  cam_mlp is the time MLP kernel with k = 3 scalars per
+// row; every block's cam_mlp.1 is one concatenated rows pass (cam_wall), as the time table's mlp.1 are.  Independent of t.
+int compute_cam(irsde_ctx* ctx, cudaStream_t st) {
+  const int n = ctx->lens_n, w = ctx->naf.width;
+  CUDA_TRY(ctx, cudaMemcpy(ctx->lens_dev, ctx->lens_host.data(), (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice));
+  launch_naf_time_gate_k(ctx->lens_dev, n, 3, w, ctx->raw["cam_mlp.0.weight"].dev, ctx->raw["cam_mlp.0.bias"].dev,
+                       ctx->raw["cam_mlp.2.weight"].dev, ctx->raw["cam_mlp.2.bias"].dev, ctx->cam_gate, st);
+  launch_time_rows(ctx->cam_gate, n, 2 * w, ctx->cam_wall, ctx->cam_ball, ctx->cam_S, ctx->cam_table, st);
+  ctx->launches += 2;
+  CUDA_TRY(ctx, cudaGetLastError());
+  return IRSDE_OK;
+}
+
+// run-time state of a lens network for a batch of B: the camera rows must be set, one shared or one per image
+int lens_ready(irsde_ctx* ctx, int B, Plan* p) {
+  p->cur.cam = nullptr;
+  p->cur.cam_img_stride = 0;
+  if (!ctx->naf.lens) return IRSDE_OK;
+  if (ctx->lens_n == 0) return fail(ctx, IRSDE_ERR_STATE, "lens network: irsde_set_lens must be called first");
+  if (ctx->lens_n != 1 && ctx->lens_n != B) return fail(ctx, IRSDE_ERR_INVALID, "lens count must be 1 or the batch size");
+  p->cur.cam = ctx->cam_table;
+  p->cur.cam_img_stride = ctx->lens_n > 1 ? 1 : 0;
   return IRSDE_OK;
 }
 
@@ -1541,6 +1607,50 @@ int irsde_create_nafnet(const irsde_nafnet_config* ncfg, irsde_ctx** out) {
   for (int i = 0; i < ncfg->n_levels; ++i) { c->naf.enc[i] = ncfg->enc_blk_nums[i]; c->naf.dec[i] = ncfg->dec_blk_nums[i]; }
   c->naf.latent = ncfg->latent != 0;
   return IRSDE_OK;
+}
+
+int irsde_create_nafnet_lens(const irsde_nafnet_config* ncfg, irsde_ctx** out) {
+  if (ncfg && ncfg->latent) return fail(nullptr, IRSDE_ERR_INVALID, "the lens network ends in a plain ending(x): latent must be 0");
+  int rc = irsde_create_nafnet(ncfg, out);
+  if (rc) return rc;
+  irsde_ctx* c = *out;
+  c->naf.lens = true;
+  int S = 0;
+  for (auto& b : naf_blocks(c->naf)) { c->cam_off[b.pre] = S; S += 2 * b.c; }
+  c->cam_S = S;
+  return IRSDE_OK;
+}
+
+int irsde_set_lens(irsde_ctx* ctx, const float* lens, int32_t n, void* stream) {
+  if (!ctx || !lens) return fail(ctx, IRSDE_ERR_INVALID, "null argument");
+  if (!ctx->naf.on || !ctx->naf.lens) return fail(ctx, IRSDE_ERR_INVALID, "irsde_set_lens: not a lens network context");
+  if (n < 1) return fail(ctx, IRSDE_ERR_INVALID, "irsde_set_lens: n must be >= 1");
+  cudaSetDevice(ctx->cfg.device);
+  std::vector<float> v(lens, lens + (size_t)n * 3);
+  if (n == ctx->lens_n && v == ctx->lens_host) return IRSDE_OK;  // the table already holds these rows
+  // captured step graphs and chains in flight on any stream read the table: drain before it is re-written or re-allocated
+  CUDA_TRY(ctx, cudaDeviceSynchronize());
+  if (n > ctx->lens_cap) {
+    for (float* q : {ctx->cam_table, ctx->cam_gate, ctx->lens_dev}) {
+      if (!q) continue;
+      auto it = std::find(ctx->allocs.begin(), ctx->allocs.end(), (void*)q);
+      if (it != ctx->allocs.end()) ctx->allocs.erase(it);
+      cudaFree(q);
+    }
+    const int cap = n < 16 ? 16 : n;
+    ctx->dev_bytes -= (long long)ctx->lens_cap * (ctx->cam_S + 2 * ctx->naf.width + 3) * 4;
+    ctx->cam_table = (float*)dev_alloc(ctx, (size_t)cap * ctx->cam_S * 4, &ctx->allocs);
+    ctx->cam_gate = (float*)dev_alloc(ctx, (size_t)cap * 2 * ctx->naf.width * 4, &ctx->allocs);
+    ctx->lens_dev = (float*)dev_alloc(ctx, (size_t)cap * 3 * 4, &ctx->allocs);
+    ctx->lens_cap = cap;
+    if (!ctx->cam_table || !ctx->cam_gate || !ctx->lens_dev) {
+      ctx->lens_cap = 0; ctx->lens_n = 0; ctx->lens_host.clear();
+      return fail(ctx, IRSDE_ERR_CUDA, "cudaMalloc camera table failed");
+    }
+  }
+  ctx->lens_host.swap(v);
+  ctx->lens_n = n;
+  return ctx->finalized ? compute_cam(ctx, (cudaStream_t)stream) : IRSDE_OK;  // else irsde_finalize_weights computes it
 }
 
 // ---- NCCL behind the C ABI (SURVEY 8 b): dlopen()ed on first use so that single-GPU users keep a library without
@@ -1743,12 +1853,14 @@ int irsde_finalize_weights(irsde_ctx* ctx) {
   // (UNet ResBlock: Linear(4nf -> 2*Cout); NAFBlock: Linear(2w -> 4c))
   struct TB { std::string pre; int rows; };
   std::vector<TB> tbs;
+  std::string mlp_name = "mlp.1.";  // the block's time Linear (lens variant: time_mlp.1)
   int td = 0;
   if (ctx->lat.on) {
     td = 1;  // no time conditioning in the autoencoder
   } else if (ctx->naf.on) {
     td = 2 * ctx->naf.width;
     for (auto& b : naf_blocks(ctx->naf)) tbs.push_back({b.pre, 4 * b.c});
+    if (ctx->naf.lens) mlp_name = "time_mlp.1.";
   } else {
     td = ctx->cfg.nf * 4;
     for (auto& rb : resblocks(ctx->cfg, ctx->udim)) tbs.push_back({rb.pre, 2 * rb.cout});
@@ -1763,9 +1875,26 @@ int irsde_finalize_weights(irsde_ctx* ctx) {
   ctx->S = S;
   for (auto& t : tbs) {
     int off = ctx->ss_off[t.pre];
-    CUDA_TRY(ctx, cudaMemcpy(ctx->wall + (size_t)off * td, ctx->raw[t.pre + "mlp.1.weight"].dev, (size_t)t.rows * td * 4,
+    CUDA_TRY(ctx, cudaMemcpy(ctx->wall + (size_t)off * td, ctx->raw[t.pre + mlp_name + "weight"].dev, (size_t)t.rows * td * 4,
                              cudaMemcpyDeviceToDevice));
-    CUDA_TRY(ctx, cudaMemcpy(ctx->ball + off, ctx->raw[t.pre + "mlp.1.bias"].dev, (size_t)t.rows * 4, cudaMemcpyDeviceToDevice));
+    CUDA_TRY(ctx, cudaMemcpy(ctx->ball + off, ctx->raw[t.pre + mlp_name + "bias"].dev, (size_t)t.rows * 4, cudaMemcpyDeviceToDevice));
+  }
+  if (ctx->naf.lens) {  // camera modulation: every block's cam_mlp.1 (Linear(2w -> 2c)) into one [cam_S][2w] matrix
+    if (!ctx->cam_wall) {
+      ctx->cam_wall = (float*)dev_alloc(ctx, (size_t)ctx->cam_S * td * 4, &ctx->allocs);
+      ctx->cam_ball = (float*)dev_alloc(ctx, (size_t)ctx->cam_S * 4, &ctx->allocs);
+      if (!ctx->cam_wall || !ctx->cam_ball) return fail(ctx, IRSDE_ERR_CUDA, "cudaMalloc failed");
+    }
+    for (auto& b : naf_blocks(ctx->naf)) {
+      const int off = ctx->cam_off[b.pre], rows = 2 * b.c;
+      CUDA_TRY(ctx, cudaMemcpy(ctx->cam_wall + (size_t)off * td, ctx->raw[b.pre + "cam_mlp.1.weight"].dev, (size_t)rows * td * 4,
+                               cudaMemcpyDeviceToDevice));
+      CUDA_TRY(ctx, cudaMemcpy(ctx->cam_ball + off, ctx->raw[b.pre + "cam_mlp.1.bias"].dev, (size_t)rows * 4, cudaMemcpyDeviceToDevice));
+    }
+    if (ctx->lens_n) {  // the table was computed from the previous weights (or not yet): recompute it
+      int rc = compute_cam(ctx, 0);
+      if (rc) return rc;
+    }
   }
   CUDA_TRY(ctx, cudaDeviceSynchronize());
   ctx->finalized = true;
@@ -1809,6 +1938,8 @@ int irsde_noise_fn(irsde_ctx* ctx, const float* x, const float* mu, const float*
   Plan* p;
   int rc = build_plan(ctx, B, H, W, &p);
   if (rc) return rc;
+  rc = lens_ready(ctx, B, p);
+  if (rc) return rc;
   CUDA_TRY(ctx, cudaMemcpyAsync(p->fwd_times, times, (size_t)n_times * 4, cudaMemcpyHostToDevice, st));
   time_rows(ctx, p->fwd_times, n_times, p->fwd_temb, p->fwd_table, st);
   p->cur.x = x; p->cur.mu = mu; p->cur.out = out;
@@ -1850,6 +1981,8 @@ int irsde_reverse(irsde_ctx* ctx, int32_t mode, const float* xT, const float* mu
   Plan* p;
   int rc = build_plan(ctx, B, H, W, &p);
   if (rc) return rc;
+  rc = lens_ready(ctx, B, p);
+  if (rc) return rc;
   long long n = (long long)B * ctx->cfg.in_nc * H * W;
   CUDA_TRY(ctx, cudaMemcpyAsync(p->x_state, xT, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
   if (mu) CUDA_TRY(ctx, cudaMemcpyAsync(p->mu_buf, mu, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
@@ -1873,6 +2006,10 @@ int irsde_reverse(irsde_ctx* ctx, int32_t mode, const float* xT, const float* mu
     ctx->launches += 2;
   };
   if (use_graph && !ctx->prof) {
+    if (p->graph[mode] && (p->graph_cam[mode] != p->cur.cam || p->graph_cam_stride[mode] != p->cur.cam_img_stride)) {
+      cudaGraphExecDestroy(p->graph[mode]);  // captured with another camera table / lens count
+      p->graph[mode] = nullptr;
+    }
     if (!p->graph[mode]) {
       cudaStream_t cs;
       CUDA_TRY(ctx, cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
@@ -1893,6 +2030,8 @@ int irsde_reverse(irsde_ctx* ctx, int32_t mode, const float* xT, const float* mu
       cudaGraphDestroy(g);
       cudaStreamDestroy(cs);
       if (e != cudaSuccess) return fail(ctx, IRSDE_ERR_CUDA, std::string("graph instantiate failed: ") + cudaGetErrorString(e));
+      p->graph_cam[mode] = p->cur.cam;
+      p->graph_cam_stride[mode] = p->cur.cam_img_stride;
     }
     for (int i = 0; i < T; ++i) CUDA_TRY(ctx, cudaGraphLaunch(p->graph[mode], st));
     ctx->launches += (long long)T * p->step_launches[mode];
@@ -2039,6 +2178,8 @@ int irsde_trace_forward(irsde_ctx* ctx, const float* x, const float* mu, const f
   if (op < 0 || op >= (int)p->ops.size()) return fail(ctx, IRSDE_ERR_INVALID, "op index out of range");
   const OpRec& r = p->ops[op];
   if (!r.out_p) return fail(ctx, IRSDE_ERR_UNSUPPORTED, "this op has no NHWC output view to read back");
+  rc = lens_ready(ctx, B, p);
+  if (rc) return rc;
   CUDA_TRY(ctx, cudaMemcpyAsync(p->fwd_times, times, (size_t)n_times * 4, cudaMemcpyHostToDevice, st));
   time_rows(ctx, p->fwd_times, n_times, p->fwd_temb, p->fwd_table, st);
   p->cur.x = x; p->cur.mu = mu; p->cur.out = p->eps_buf;

@@ -3,7 +3,7 @@
 // All are HBM-bound NHWC kernels (fp32 math; float or bf16 storage).
 #include <math.h>
 
-#include "common.cuh"
+#include "nafnet.cuh"
 
 namespace irsde {
 
@@ -115,15 +115,55 @@ __global__ void scale_channels_kernel(T* __restrict__ x, int pitch, const float*
 }
 
 // SimpleGate on a [.., 2c] tensor -> [.., c]                                   (:9-12)
+// cam != null: the lens network's per-image FFN modulation follows the gate
+//   g = (a*b) * (cam_scale[img][ch] + 1) + cam_shift[img][ch]      (latent-bokeh/.../DenoisingNAFNet_arch.py:82-83)
+// in fp32 with the reference's separate roundings (mul, then add), stored once as T.
 template <typename T>
-__global__ void simple_gate_kernel(const T* __restrict__ x, int x_pitch, T* __restrict__ out, int o_pitch, long long npix, int c) {
+__global__ void simple_gate_kernel(const T* __restrict__ x, int x_pitch, T* __restrict__ out, int o_pitch, long long npix, int c,
+                                   CamMod cm) {
   PDL_ENTRY();
   long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   long long total = npix * c;
   if (idx >= total) return;
   const int ch = idx % c;
   const long long p = idx / c;
-  out[p * o_pitch + ch] = from_f<T>(to_f(x[p * x_pitch + ch]) * to_f(x[p * x_pitch + ch + c]));
+  float v = to_f(x[p * x_pitch + ch]) * to_f(x[p * x_pitch + ch + c]);
+  if (cm.cam) {
+    const float* r = cm.cam + (long long)(p / cm.pix_per_img) * cm.img_stride * cm.S + cm.off;
+    v = __fadd_rn(__fmul_rn(v, __fadd_rn(r[ch], 1.f)), r[c + ch]);
+  }
+  out[p * o_pitch + ch] = from_f<T>(v);
+}
+
+// 16-byte vector loads/stores of the same modulated gate: grid (pixel groups, 1, image), block (channel vectors, pixels);
+// needs c % VEC == 0 (VEC = 16 bytes of T) and 16-byte aligned views.  No per-element index arithmetic.
+template <typename T>
+struct alignas(16) Vec16 {
+  static constexpr int N = 16 / sizeof(T);
+  T v[N];
+};
+template <typename T>
+__global__ void __launch_bounds__(256) simple_gate_cam_vec_kernel(const T* __restrict__ x, int x_pitch, T* __restrict__ out,
+                                                                  int o_pitch, int N, int c, CamMod cm) {
+  PDL_ENTRY();
+  constexpr int VEC = Vec16<T>::N;
+  const int pix = blockIdx.x * blockDim.y + threadIdx.y;
+  if (pix >= N) return;
+  const long long p = (long long)blockIdx.z * N + pix;
+  const float* r = cm.cam + (long long)blockIdx.z * cm.img_stride * cm.S + cm.off;
+  const T* xa = x + p * x_pitch;
+  T* o = out + p * o_pitch;
+  for (int j = threadIdx.x * VEC; j < c; j += blockDim.x * VEC) {
+    const Vec16<T> a = *reinterpret_cast<const Vec16<T>*>(xa + j);
+    const Vec16<T> b = *reinterpret_cast<const Vec16<T>*>(xa + c + j);
+    Vec16<T> g;
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) {
+      const float v = to_f(a.v[e]) * to_f(b.v[e]);
+      g.v[e] = from_f<T>(__fadd_rn(__fmul_rn(v, __fadd_rn(r[j + e], 1.f)), r[c + j + e]));
+    }
+    *reinterpret_cast<Vec16<T>*>(o + j) = g;
+  }
 }
 
 // PixelShuffle(2) of a [B,h,w,4q] tensor + skip add -> [B,2h,2w,q]              (:132-137,172-174)
@@ -201,11 +241,31 @@ template void launch_scale_channels<bf16>(bf16*, int, const float*, int, int, in
 
 template <typename T>
 void launch_simple_gate(const T* x, int x_pitch, T* out, int o_pitch, long long npix, int c, cudaStream_t st) {
+  CamMod none;
+  memset(&none, 0, sizeof none);
   long long total = npix * c;
-  pdl_launch(simple_gate_kernel<T>, (unsigned)((total + 255) / 256), 256, 0, st, x, x_pitch, out, o_pitch, npix, c);
+  pdl_launch(simple_gate_kernel<T>, (unsigned)((total + 255) / 256), 256, 0, st, x, x_pitch, out, o_pitch, npix, c, none);
 }
 template void launch_simple_gate<float>(const float*, int, float*, int, long long, int, cudaStream_t);
 template void launch_simple_gate<bf16>(const bf16*, int, bf16*, int, long long, int, cudaStream_t);
+
+template <typename T>
+void launch_simple_gate(const T* x, int x_pitch, T* out, int o_pitch, long long npix, int c, cudaStream_t st, const CamMod& cam,
+                        int B) {
+  constexpr int VEC = Vec16<T>::N;
+  const bool aligned = ((uintptr_t)x % 16 == 0) && ((uintptr_t)out % 16 == 0) && x_pitch % VEC == 0 && o_pitch % VEC == 0;
+  if (cam.cam && c % VEC == 0 && aligned) {
+    const int cv = c / VEC, bx = cv < 256 ? cv : 256, by = 256 / bx;
+    const int N = (int)(npix / B);
+    pdl_launch(simple_gate_cam_vec_kernel<T>, dim3((N + by - 1) / by, 1, B), dim3(bx, by), 0, st, x, x_pitch, out, o_pitch, N, c,
+               cam);
+    return;
+  }
+  long long total = npix * c;
+  pdl_launch(simple_gate_kernel<T>, (unsigned)((total + 255) / 256), 256, 0, st, x, x_pitch, out, o_pitch, npix, c, cam);
+}
+template void launch_simple_gate<float>(const float*, int, float*, int, long long, int, cudaStream_t, const CamMod&, int);
+template void launch_simple_gate<bf16>(const bf16*, int, bf16*, int, long long, int, cudaStream_t, const CamMod&, int);
 
 template <typename T>
 void launch_pixel_shuffle_add(const T* in, int in_pitch, const T* skip, int s_pitch, T* out, int o_pitch, int B, int h, int w, int q,
@@ -228,43 +288,52 @@ template void launch_add<bf16>(const bf16*, int, const bf16*, int, bf16*, int, l
 // NAFNet timestep embedding: SinusoidalPosEmb(w) -> Linear(w, 8w) -> SimpleGate -> Linear(4w, 4w) = t;
 // every NAFBlock: SimpleGate(t) -> Linear(2w, 4c) -> (shift_att, scale_att, shift_ffn, scale_ffn)
 // (DenoisingNAFNet_arch.py:18-20,51-54,96-101).  Stores SimpleGate(t) [2w] per row for time_table_kernel.
+// A row holds k scalars: the embedding is [sin, cos] of each, concatenated in order (k*w inputs to the first Linear).
+// k = 3 is the lens network's camera embedding cat(SinusoidalPosEmb(w)(src_lens, tgt_lens, disparity)) -> cam_mlp
+// (latent-bokeh/models/modules/DenoisingNAFNet_arch.py:109-114,171-173); k = 1 is the time path.
 // =============================================================================================
-__global__ void naf_time_mlp_kernel(const float* __restrict__ times, int width, const float* __restrict__ w1,
+__global__ void naf_time_mlp_kernel(const float* __restrict__ times, int k, int width, const float* __restrict__ w1,
                                     const float* __restrict__ b1, const float* __restrict__ w2, const float* __restrict__ b2,
                                     float* __restrict__ tgate) {
   extern __shared__ float sm[];
-  const int td = width * 4, half = width / 2;
-  float* emb = sm;            // [w]
-  float* h1 = sm + width;     // [8w]
+  const int td = width * 4, half = width / 2, kw = k * width;
+  float* emb = sm;            // [k*w]
+  float* h1 = sm + kw;        // [8w]
   float* tt = h1 + 2 * td;    // [4w]
   const int row = blockIdx.x;
-  const float t = times[row];
   const float e = logf(10000.0f) / (float)(half - 1);
-  for (int i = threadIdx.x; i < half; i += blockDim.x) {
-    const float a = t * expf((float)i * -e);
-    emb[i] = sinf(a);
-    emb[half + i] = cosf(a);
+  for (int j = 0; j < k; ++j) {
+    const float t = times[row * k + j];
+    for (int i = threadIdx.x; i < half; i += blockDim.x) {
+      const float a = t * expf((float)i * -e);
+      emb[j * width + i] = sinf(a);
+      emb[j * width + half + i] = cosf(a);
+    }
   }
   __syncthreads();
   for (int o = threadIdx.x; o < 2 * td; o += blockDim.x) {
     float s = 0.f;
-    for (int k = 0; k < width; ++k) s += w1[o * width + k] * emb[k];
+    for (int q = 0; q < kw; ++q) s += w1[o * kw + q] * emb[q];
     h1[o] = s + b1[o];
   }
   __syncthreads();
   for (int o = threadIdx.x; o < td; o += blockDim.x) {
     float s = 0.f;
-    for (int k = 0; k < td; ++k) s += w2[o * td + k] * (h1[k] * h1[k + td]);
+    for (int q = 0; q < td; ++q) s += w2[o * td + q] * (h1[q] * h1[q + td]);
     tt[o] = s + b2[o];
   }
   __syncthreads();
   for (int o = threadIdx.x; o < td / 2; o += blockDim.x) tgate[(long long)row * (td / 2) + o] = tt[o] * tt[o + td / 2];
 }
 
+void launch_naf_time_gate_k(const float* times, int rows, int k, int width, const float* w1, const float* b1, const float* w2,
+                            const float* b2, float* tgate, cudaStream_t st) {
+  const int td = width * 4;
+  naf_time_mlp_kernel<<<rows, 256, (k * width + 2 * td + td) * sizeof(float), st>>>(times, k, width, w1, b1, w2, b2, tgate);
+}
 void launch_naf_time_gate(const float* times, int rows, int width, const float* w1, const float* b1, const float* w2,
                           const float* b2, float* tgate, cudaStream_t st) {
-  const int td = width * 4;
-  naf_time_mlp_kernel<<<rows, 256, (width + 2 * td + td) * sizeof(float), st>>>(times, width, w1, b1, w2, b2, tgate);
+  launch_naf_time_gate_k(times, rows, 1, width, w1, b1, w2, b2, tgate, st);
 }
 
 }  // namespace irsde

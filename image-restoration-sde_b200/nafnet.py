@@ -1,6 +1,8 @@
 """``ConditionalNAFNet`` (Refusion's score network) with the reference's constructor, ``forward(inp, cond, time)``
 signature and state-dict names/shapes (codes/config/deraining/models/modules/DenoisingNAFNet_arch.py:87-188; latent
-variant codes/config/latent-dehazing/models/modules/DenoisingNAFNet_arch.py:147-181), executed by the native library.
+variant codes/config/latent-dehazing/models/modules/DenoisingNAFNet_arch.py:147-181; lens-conditioned variant
+codes/config/latent-bokeh/models/modules/DenoisingNAFNet_arch.py:93-199, ``forward(inp, cond, time, lens_info=...)``),
+executed by the native library.
 """
 import ctypes
 
@@ -11,14 +13,22 @@ from . import _lib
 from .unet import ConditionalUNet, _Node
 
 
-def nafnet_param_shapes(img_channel, width, middle_blk_num, enc_blk_nums, dec_blk_nums):
-    """State-dict entries in the reference's registration order (DenoisingNAFNet_arch.py:15-49,89-143)."""
+def nafnet_param_shapes(img_channel, width, middle_blk_num, enc_blk_nums, dec_blk_nums, lens=False):
+    """State-dict entries in the reference's registration order (DenoisingNAFNet_arch.py:15-49,89-143).  ``lens``: the
+    latent-bokeh variant (latent-bokeh/.../DenoisingNAFNet_arch.py:18-24,102-113): ``time_mlp.0/.2`` and ``cam_mlp.0/.2`` at
+    the top, ``time_mlp.1`` and ``cam_mlp.1`` in every block."""
     S = {}
     td = width * 4
-    S["time_mlp.1.weight"] = (td * 2, width)
-    S["time_mlp.1.bias"] = (td * 2,)
-    S["time_mlp.3.weight"] = (td, td)
-    S["time_mlp.3.bias"] = (td,)
+    t1, t3 = ("time_mlp.0.", "time_mlp.2.") if lens else ("time_mlp.1.", "time_mlp.3.")
+    S[t1 + "weight"] = (td * 2, width)
+    S[t1 + "bias"] = (td * 2,)
+    S[t3 + "weight"] = (td, td)
+    S[t3 + "bias"] = (td,)
+    if lens:
+        S["cam_mlp.0.weight"] = (td * 2, width * 3)
+        S["cam_mlp.0.bias"] = (td * 2,)
+        S["cam_mlp.2.weight"] = (td, td)
+        S["cam_mlp.2.bias"] = (td,)
     S["intro.weight"] = (width, img_channel * 2, 3, 3)
     S["intro.bias"] = (width,)
     S["ending.weight"] = (img_channel, width, 3, 3)
@@ -27,8 +37,12 @@ def nafnet_param_shapes(img_channel, width, middle_blk_num, enc_blk_nums, dec_bl
     def blk(pre, c):
         S[pre + "beta"] = (1, c, 1, 1)
         S[pre + "gamma"] = (1, c, 1, 1)
-        S[pre + "mlp.1.weight"] = (4 * c, td // 2)
-        S[pre + "mlp.1.bias"] = (4 * c,)
+        mlp = pre + ("time_mlp.1." if lens else "mlp.1.")
+        S[mlp + "weight"] = (4 * c, td // 2)
+        S[mlp + "bias"] = (4 * c,)
+        if lens:
+            S[pre + "cam_mlp.1.weight"] = (2 * c, td // 2)
+            S[pre + "cam_mlp.1.bias"] = (2 * c,)
         for name, shp in (("conv1", (2 * c, c, 1, 1)), ("conv2", (2 * c, 1, 3, 3)), ("conv3", (c, c, 1, 1)),
                           ("sca.1", (c, c, 1, 1)), ("conv4", (2 * c, c, 1, 1)), ("conv5", (c, c, 1, 1))):
             S[pre + name + ".weight"] = shp
@@ -68,30 +82,36 @@ class _NafConfig(ctypes.Structure):
 
 
 class _NafContext(_lib.Context):
-    def __init__(self, img_channel, width, middle, enc, dec, latent, precision, device_index, force_simt=False):
+    def __init__(self, img_channel, width, middle, enc, dec, latent, precision, device_index, force_simt=False, lens=False):
         L = _lib.load()
-        L.irsde_create_nafnet.argtypes = [ctypes.POINTER(_NafConfig), ctypes.POINTER(ctypes.c_void_p)]
-        L.irsde_create_nafnet.restype = ctypes.c_int
+        create = L.irsde_create_nafnet_lens if lens else L.irsde_create_nafnet
+        create.argtypes = [ctypes.POINTER(_NafConfig), ctypes.POINTER(ctypes.c_void_p)]
+        create.restype = ctypes.c_int
         cfg = _NafConfig(img_channel, width, middle, len(enc), (ctypes.c_int32 * 8)(*enc), (ctypes.c_int32 * 8)(*dec),
                          1 if latent else 0, precision, device_index, 1 if force_simt else 0)
         h = ctypes.c_void_p()
-        _lib.check(L.irsde_create_nafnet(ctypes.byref(cfg), ctypes.byref(h)))
+        _lib.check(create(ctypes.byref(cfg), ctypes.byref(h)))
         self.h = h
         self.L = L
 
 
 class ConditionalNAFNet(ConditionalUNet):
     """Drop-in for the reference ``ConditionalNAFNet``.  ``latent=True`` selects the latent-dehazing variant
-    (``ending(x + intro(x))``).  Inherits weight upload / forward plumbing from ``ConditionalUNet``."""
+    (``ending(x + intro(x))``); ``lens=True`` the latent-bokeh variant, whose blocks are also modulated by a camera
+    embedding of ``lens_info = [src_lens, tgt_lens, disparity]`` (``forward(inp, cond, time, lens_info=...)``).
+    Inherits weight upload / forward plumbing from ``ConditionalUNet``."""
 
     variant = "conditional"
 
     def __init__(self, img_channel=3, width=16, middle_blk_num=1, enc_blk_nums=[], dec_blk_nums=[], upscale=1,
-                 latent=False, precision=None, force_simt=False):
+                 latent=False, precision=None, force_simt=False, lens=False):
         nn.Module.__init__(self)
         import os
         if len(enc_blk_nums) != len(dec_blk_nums) or len(enc_blk_nums) > 8:
             raise ValueError("enc_blk_nums / dec_blk_nums must have the same length (<= 8)")
+        if lens and latent:
+            raise ValueError("the lens network ends in a plain ending(x): latent must be False")
+        self.lens = bool(lens)
         self.in_nc = self.out_nc = img_channel
         self.img_channel, self.width, self.middle_blk_num = img_channel, width, middle_blk_num
         self.enc_blk_nums, self.dec_blk_nums = list(enc_blk_nums), list(dec_blk_nums)
@@ -100,7 +120,7 @@ class ConditionalNAFNet(ConditionalUNet):
         if self.precision not in _lib.PRECISIONS:
             raise ValueError("precision must be one of %s" % (sorted(_lib.PRECISIONS),))
         self._force_simt = force_simt
-        self._shapes = nafnet_param_shapes(img_channel, width, middle_blk_num, enc_blk_nums, dec_blk_nums)
+        self._shapes = nafnet_param_shapes(img_channel, width, middle_blk_num, enc_blk_nums, dec_blk_nums, self.lens)
         for name, shp in self._shapes.items():
             parts = name.split(".")
             node = self
@@ -126,11 +146,44 @@ class ConditionalNAFNet(ConditionalUNet):
                 self._ctx.close()
             self._ctx = _NafContext(self.img_channel, self.width, self.middle_blk_num, self.enc_blk_nums, self.dec_blk_nums,
                                     self.latent, _lib.PRECISIONS[self.precision], idx,
-                                    force_simt=self._force_simt)
+                                    force_simt=self._force_simt, lens=self.lens)
             self._ctx_dev = idx
             self._sig = None
         return self._ctx
 
+    @staticmethod
+    def lens_rows(lens_info):
+        """``[src_lens, tgt_lens, disparity]`` -> host float32 ``[n][3]``.  Each entry is a Python number, a 1-element tensor
+        (what the DataLoader yields at batch 1) or an ``[n]`` tensor, on any device; 1-element entries are shared by the
+        batch."""
+        if len(lens_info) != 3:
+            raise ValueError("lens_info must hold 3 entries [src_lens, tgt_lens, disparity], got %d" % len(lens_info))
+        cols = [torch.as_tensor(v).detach().reshape(-1).float().cpu() for v in lens_info]
+        n = max(c.numel() for c in cols)
+        if any(c.numel() not in (1, n) for c in cols):
+            raise ValueError("lens_info entries must hold 1 or the same number of values")
+        return torch.stack([c.expand(n) for c in cols], dim=1).contiguous()
+
+    def set_lens(self, lens_info, device):
+        """Camera rows of the following forwards / chains on ``device`` (irsde_set_lens): one row shared by the batch, or one
+        per image, where image b's result is the network run on image b alone with its own lens."""
+        self._upload_lens(self.lens_rows(lens_info), device)
+
+    def _upload_lens(self, rows, device):
+        ctx = self.sync_weights(device)
+        arr = _lib.float_array(rows.reshape(-1).tolist())
+        with torch.cuda.device(device):
+            st = torch.cuda.current_stream().cuda_stream
+            _lib.check(ctx.L.irsde_set_lens(ctx.h, arr, rows.shape[0], ctypes.c_void_p(st)), ctx.h)
+
     @torch.no_grad()
-    def forward(self, inp, cond, time):
+    def forward(self, inp, cond, time, **kwargs):
+        if not self.lens:
+            if kwargs:
+                raise TypeError("forward() got an unexpected keyword argument %r" % next(iter(kwargs)))
+            return self._run(inp, cond, time)
+        rows = self.lens_rows(kwargs["lens_info"])  # KeyError('lens_info') without it, as the reference (:161)
+        if not inp.is_cuda:
+            raise RuntimeError("irsde_b200.ConditionalNAFNet runs on CUDA (sm_100a) only; there is no CPU path")
+        self._upload_lens(rows, inp.device)
         return self._run(inp, cond, time)

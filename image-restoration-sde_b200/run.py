@@ -10,7 +10,9 @@ What it does before handing control to the script (nothing in the reference tree
     (codes/utils/sde_utils.py:80,373) - every other helper (img/file/deg utils) stays the reference's;
   * import the task's ``models.modules`` and swap ``ConditionalUNet`` for ours (the factory is
     ``getattr(M, which_model_G)(**setting)``, models/networks.py:10-15), choosing the variant by the
-    reference class's own ``forward`` signature (``(x, time)`` => denoising-sde variant);
+    reference class's own ``forward`` signature (``(x, time)`` => denoising-sde variant); likewise
+    ``ConditionalNAFNet``: a ``forward`` taking ``**kwargs`` => the lens-conditioned latent-bokeh network
+    (``lens=True``), otherwise ``latent=True`` when the task directory's name contains "latent";
   * provide tiny stand-ins for optional third-party modules the scripts import but this image lacks
     (IPython.embed, lpips.LPIPS, lmdb, ema_pytorch.EMA) - only when the real ones are not importable.
 
@@ -97,9 +99,16 @@ def install(script_dir):
             ours = irsde_b200.DenoisingUNet
     mods.ConditionalUNet = ours
     if hasattr(mods, "ConditionalNAFNet"):
-        latent = "latent" in os.path.basename(os.path.abspath(script_dir))
         import functools
-        mods.ConditionalNAFNet = functools.partial(irsde_b200.ConditionalNAFNet, latent=latent) if latent else irsde_b200.ConditionalNAFNet
+        ref_naf = mods.ConditionalNAFNet
+        if not (isinstance(ref_naf, functools.partial) or ref_naf is irsde_b200.ConditionalNAFNet):  # not installed yet
+            kinds = [p.kind for p in inspect.signature(ref_naf.forward).parameters.values()]
+            if inspect.Parameter.VAR_KEYWORD in kinds:  # forward(inp, cond, time, **kwargs): latent-bokeh's lens network
+                mods.ConditionalNAFNet = functools.partial(irsde_b200.ConditionalNAFNet, lens=True)
+            else:
+                latent = "latent" in os.path.basename(os.path.abspath(script_dir))
+                mods.ConditionalNAFNet = (functools.partial(irsde_b200.ConditionalNAFNet, latent=latent) if latent
+                                          else irsde_b200.ConditionalNAFNet)
     if hasattr(mods, "UNet"):
         mods.UNet = irsde_b200.UNet
     return utils, mods

@@ -178,10 +178,13 @@ class _SDEBase:
                                         ctypes.c_void_p(st)), ctx.h)
         return out
 
-    def _native_chain(self, mode, xt, mu, T, zs=None):
-        """Whole loop in the library: T network forwards + T fused updates (one captured step graph)."""
+    def _native_chain(self, mode, xt, mu, T, zs=None, lens_info=None):
+        """Whole loop in the library: T network forwards + T fused updates (one captured step graph).  ``lens_info``: the
+        lens network's camera rows, set once for the chain (they do not depend on t)."""
         m = _unwrap(self.model)
         ctx = self._ctx_for(xt)
+        if lens_info is not None:
+            m.set_lens(lens_info, xt.device)
         x = xt.contiguous().float()
         B, C, H, W = x.shape
         if mu is not None:
@@ -208,7 +211,11 @@ class _SDEBase:
 
     def _fast(self, kwargs, save_states):
         m = _unwrap(self.model) if self.model is not None else None
-        return isinstance(m, ConditionalUNet) and not kwargs and not save_states
+        if not isinstance(m, ConditionalUNet) or save_states:
+            return False
+        if getattr(m, "lens", False):  # the lens network's one keyword: set once per chain; without it the loop raises KeyError
+            return set(kwargs) == {"lens_info"}
+        return not kwargs
 
     @staticmethod
     def _save(x, t, T_total, save_dir):
@@ -283,7 +290,7 @@ class IRSDE(_SDEBase):
     def _loop(self, mode, name, xt, T, save_states, save_dir, kwargs, zs=None):
         T = self.T if T < 0 else T
         if self._fast(kwargs, save_states):
-            return self._native_chain(mode, xt, self.mu, T, zs)
+            return self._native_chain(mode, xt, self.mu, T, zs, kwargs.get("lens_info"))
         x = xt.clone()
         for i, t in enumerate(reversed(range(1, T + 1))):
             noise = self.noise_fn(x, t, **kwargs)

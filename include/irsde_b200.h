@@ -107,6 +107,16 @@ int irsde_create_ch_mult(const irsde_config* cfg, const int32_t* ch_mult, int32_
 /* Same context type, ConditionalNAFNet architecture; every other entry point (load_tensor, noise_fn, reverse, ...)
  * is shared.  Replaces `ConditionalNAFNet(...)` + `.to(device)` (DenoisingNAFNet_arch.py:89). */
 int irsde_create_nafnet(const irsde_nafnet_config* cfg, irsde_ctx** out);
+/* ConditionalNAFNet of codes/config/latent-bokeh (models/modules/DenoisingNAFNet_arch.py:92-200): time + camera-conditioned
+ * blocks, plain ending(x); cfg->latent must be 0.  State-dict names: time_mlp.0/.2 and cam_mlp.0/.2 at the top, time_mlp.1 and
+ * cam_mlp.1 in every block.  Every run (noise_fn, reverse, trace_forward) needs irsde_set_lens first (IRSDE_ERR_STATE). */
+int irsde_create_nafnet_lens(const irsde_nafnet_config* cfg, irsde_ctx** out);
+/* lens: HOST [n][3] = (src_lens, tgt_lens, disparity) per image as the dataset yields them; n = 1 (shared) or the B of the
+ * following noise_fn / reverse / trace_forward calls (else those return IRSDE_ERR_INVALID).  Computes the per-image camera
+ * rows on the device (cam_mlp, then every block's cam_mlp.1): once per call, not per step.  Drains the device before it
+ * re-writes the rows, so a chain already enqueued keeps the lens it was started with.  IRSDE_ERR_INVALID on a context that
+ * is not a lens network. */
+int irsde_set_lens(irsde_ctx* ctx, const float* lens, int32_t n, void* stream);
 void irsde_destroy(irsde_ctx* ctx);
 const char* irsde_last_error(const irsde_ctx* ctx);
 /* "irsde_b200 <version> sm_100a" */
